@@ -18,6 +18,7 @@ Extra objects in the same JSON line (each timed the same way: CUDA events, max o
   python bench.py --gpus 1 --steps 10 --warmup 3
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference        # CPU restatement of the reference (oracle/) on the host cores, same workload
+  python bench.py --dump-outputs DIR      # also save what the last timed step returned (seeded clip sample) as DIR/*.npy
 """
 import argparse
 import json
@@ -27,6 +28,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the source tree, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -41,6 +43,7 @@ DEFAULT_CLIPS = 296          # clips per GPU = 2 x 148 SMs (each clip is 4 tiles
 GEN_MACS, FNET_MACS = 1420992, 126720
 WORKLOAD = ("metric config: 4x SR inference of synthetic 10-frame clips 32x32->128x128, %d clips per GPU in lock-step "
             "(generator N=16 + fnet, full recurrence)")
+DUMP_CLIPS = 16              # --dump-outputs: 16 of the clips, 10 x 16 HR frames as float32 = 31 MB (all 296 would be 582 MB)
 
 
 def clip_flop(T=CLIP_T, px=LR * LR):
@@ -210,7 +213,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip configs[1], the config-5 sweep and the training steps")
     ap.add_argument("--train-steps", type=int, default=4)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save what the headline path returned in its last step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -356,6 +363,9 @@ def main():
     note("headline: resident %.2f ms/step, e2e %.2f ms/step" % (ms_res / args.steps, ms_e2e / args.steps))
     # the e2e leg really moved the bytes: spot-check the host copy against the device result of the last batch
     assert torch.equal(host_out[(args.steps - 1) & 1][-1, 0], eng.clip_u8[-1, 0].cpu()), "e2e: host frames differ from device frames"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, host_out[(args.steps - 1) & 1], eng.out01)
+        note("outputs of the last timed step written to %s" % args.dump_outputs)
 
     # --- dominant kernel: the generator trunk (input conv + 16 residual blocks = 33 layers of 3x3 64->64) on the whole clip
     # batch [B,32,32,64] -- ONE launch of conv3x3_lin_kernel (kx-fused N=192 MMAs, CTA-local clips) -- timed alone (graph replay).
@@ -528,6 +538,19 @@ def main():
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, frames_u8, last_f32):
+    """Save what a ClipEngine caller received from one clip batch, for a fixed seeded sample of the clips, so that two builds
+    can be compared output for output: hr_frames_u8 [T,S,128,128,3] (the uint8 HR frames as float32), hr_last_frame_f32
+    [S,128,128,3] (fp32 output of the last frame) and sample_clips [S] (the clip indices, float64)."""
+    B = frames_u8.shape[1]
+    idx = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_CLIPS), replace=False))
+    sel = torch.from_numpy(idx)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "hr_frames_u8.npy"), frames_u8[:, sel].float().numpy())
+    np.save(os.path.join(out_dir, "hr_last_frame_f32.npy"), last_f32[sel.to(last_f32.device)].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "sample_clips.npy"), idx.astype(np.float64))
 
 
 def _traffic(name):

@@ -264,3 +264,26 @@ def test_conv_transpose_gradients_through_the_space_to_depth_identity():
     (dx * x.detach()).sum().backward()            # d/dW' of sum_p conv(dzs, W')[p] . x[p]  =  the wgrad kernel's sum
     dw = wp.grad.view(36, C, C).index_select(0, idx).view(3, 3, C, C)
     assert (dw - w.grad).abs().max().item() < 1e-4 * max(1.0, w.grad.abs().max().item())
+
+
+def test_bench_dump_outputs_is_a_small_seeded_float_sample(tmp_path):
+    """bench.py --dump-outputs: for the metric configuration's clip batch (296 clips x 10 frames of 128x128 uint8) the
+    files are float32 / float64, hold the same seeded clips on every run, and stay below 64 MB in all."""
+    import bench
+    T, B = bench.CLIP_T, bench.DEFAULT_CLIPS
+    u8 = (torch.arange(B) % 256).to(torch.uint8).view(1, B, 1, 1, 1).expand(T, B, 4 * bench.LR, 4 * bench.LR, 3).contiguous()
+    last = torch.arange(B, dtype=torch.float32).view(B, 1, 1, 1).expand(B, 4 * bench.LR, 4 * bench.LR, 3).contiguous()
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), u8, last)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["hr_frames_u8.npy", "hr_last_frame_f32.npy", "sample_clips.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 * 2 ** 20
+    a = {n: np.load(tmp_path / "a" / n) for n in names}
+    for n in names:
+        assert a[n].dtype in (np.float32, np.float64)
+        np.testing.assert_array_equal(a[n], np.load(tmp_path / "b" / n))
+    idx = a["sample_clips.npy"].astype(np.int64)
+    assert len(set(idx.tolist())) == len(idx) == bench.DUMP_CLIPS and idx.max() < B
+    assert a["hr_frames_u8.npy"].shape == (T, len(idx), 128, 128, 3)
+    np.testing.assert_array_equal(a["hr_frames_u8.npy"][:, :, 0, 0, 0], np.broadcast_to(idx % 256, (T, len(idx))))
+    np.testing.assert_array_equal(a["hr_last_frame_f32.npy"][:, 5, 7, 1], idx)
