@@ -23,6 +23,42 @@ int teco_sm_count() {
   return sms;
 }
 
+int teco_tmap_bf16(CUtensorMap* map, const char* who, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                   const cuuint32_t* box) {
+  typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  static EncodeTiled enc = nullptr;
+  if (!enc) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
+        qres == cudaDriverEntryPointSuccess)
+      enc = (EncodeTiled)p;
+  }
+  if (!enc) {
+    teco_set_error("%s: cuTensorMapEncodeTiled is unavailable (no CUDA driver?)", who);
+    return TECO_E_CUDA;
+  }
+  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  const CUresult cr = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
+                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (cr != CUDA_SUCCESS) {
+    teco_set_error("%s: cuTensorMapEncodeTiled failed with CUresult %d (rank %d, innermost dimensions %llu x %llu)", who, (int)cr, rank,
+                   (unsigned long long)dims[0], (unsigned long long)dims[1]);
+    return TECO_E_CUDA;
+  }
+  return TECO_OK;
+}
+
+int teco_tmap_nhwc(CUtensorMap* map, const char* who, const void* base, int N, int H, int W, int C, int box_c, int box_w, int box_h) {
+  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+  const cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
+  const cuuint32_t box[4] = {(cuuint32_t)box_c, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
+  return teco_tmap_bf16(map, who, base, 4, dims, strides, box);
+}
+
 extern "C" {
 
 const char* teco_last_error(void) { return g_err; }

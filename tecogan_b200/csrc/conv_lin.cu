@@ -396,22 +396,6 @@ conv3x3_lin_kernel(const __grid_constant__ LinMaps maps, const LinParams p) {
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
-  return fn;
-}
-
 }  // namespace
 
 extern long long* teco_g_dbg_timing;   // conv_tc.cu
@@ -448,28 +432,11 @@ extern "C" int teco_conv3x3_lin_tc(int32_t N, int32_t H, int32_t W, int32_t num_
   const int sms = teco_sm_count();
   p.G = N < sms ? N : sms;
 
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) {
-    teco_set_error("teco_conv3x3_lin_tc: cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
-    return TECO_E_CUDA;
-  }
   LinMaps maps;
-  const cuuint64_t gdim[4] = {64, (cuuint64_t)LW, (cuuint64_t)H, (cuuint64_t)N};
-  const cuuint64_t gstr[3] = {128, (cuuint64_t)LW * 128, (cuuint64_t)H * LW * 128};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
   for (int i = 0; i < 3; ++i) {
     void* base = bufs[i] ? bufs[i] : bufs[1] ? bufs[1] : bufs[0];   // an unused slot still needs a valid map
-    const cuuint32_t box_ld[4] = {64, (cuuint32_t)LW, (cuuint32_t)HALO_ROWS, 1};
-    const cuuint32_t box_st[4] = {64, (cuuint32_t)LW, (cuuint32_t)STRIP_ROWS, 1};
-    CUresult cr = enc(&maps.ld[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, gdim, gstr, box_ld, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr == CUDA_SUCCESS)
-      cr = enc(&maps.st[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, gdim, gstr, box_st, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) {
-      teco_set_error("teco_conv3x3_lin_tc: cuTensorMapEncodeTiled failed with CUresult %d (N=%d H=%d)", (int)cr, N, H);
-      return TECO_E_CUDA;
-    }
+    if (int e = teco_tmap_nhwc(&maps.ld[i], "teco_conv3x3_lin_tc", base, N, H, LW, 64, 64, LW, HALO_ROWS)) return e;
+    if (int e = teco_tmap_nhwc(&maps.st[i], "teco_conv3x3_lin_tc", base, N, H, LW, 64, 64, LW, STRIP_ROWS)) return e;
   }
   TECO_CUDA_CALL(cudaFuncSetAttribute(conv3x3_lin_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
   cudaLaunchConfig_t cfg = {};

@@ -8,14 +8,15 @@
 // Implicit GEMM, no im2col buffer:
 //   CTA tile  = 16 image rows x (8*J) pixels; every 16x8 sub-tile is one UMMA accumulator with M = 128.
 //   A operand = NHWC bf16 activations, 64 channels = one 128-byte row per pixel.  Per 64-channel block the halo is
-//               staged by THREE 4-D TMA boxes (64 ch, 8J px, 18 rows, 1 image), one per horizontal tap offset kx,
-//               with SWIZZLE_128B.  Each box is the UMMA canonical K-major SW128 layout as it lands
-//               (8 consecutive pixels = one 1024-byte swizzle atom, SBO = one box row).  Vertical taps ky are
-//               descriptor start-address offsets of whole box rows (atom aligned), so 3 loads serve 9 taps.
-//               TMA out-of-bounds zero fill implements TF 'SAME' padding.
+//               staged by ONE 4-D TMA box (64 ch, 8J+2 px, 18 rows, 1 image) with SWIZZLE_128B, which is the UMMA
+//               canonical K-major SW128 layout as it lands (SBO = one box row).  All nine taps are descriptor start
+//               offsets into it: vertical taps ky whole box rows, horizontal taps kx 128-byte pixel rows (not
+//               swizzle-atom aligned: the SW128 XOR is a function of the absolute shared-memory address bits, which is
+//               also how TMA wrote the box; the descriptor's base-offset field stays 0 -- setting it to (addr >> 7) & 7
+//               was tested on the B200 and gives wrong results).  TMA out-of-bounds zero fill implements TF 'SAME' padding.
 //   B operand = weights pre-packed on the device as [cin/64][tap][cout][64 cin] bf16 in the same SW128 image,
 //               streamed by 1-D bulk copies.  When a whole layer fits (64->64: 72 KB) the slabs are fetched once,
-//               BEFORE the programmatic-dependent-launch wait, and multicast across a 4-CTA cluster.
+//               BEFORE the programmatic-dependent-launch wait (the one-tile kernel also multicasts them over a 4-CTA cluster).
 //   D         = fp32 in TMEM, column block (sub-tile, phase) * Cout.
 // Transposed conv (stride 2, TF 'SAME', y[i] = sum_j x[j] w[i-2j]) is the same loop with the nine taps routed to
 // four sub-pixel phase accumulators (SURVEY.md A.3) and a 2x interleaving epilogue.
@@ -25,20 +26,12 @@
 //
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2..9 = epilogue
 // (one epilogue warp per scheduler is latency-bound: ~1000 clk per 32 channels; two per scheduler halve it).
-#include <cuda.h>
-#include <cstdlib>
 #include <type_traits>
-#include "teco_common.cuh"
-#include "tc_ptx.cuh"
+#include "conv_tc_common.cuh"
 
 namespace {
 
-constexpr int TILE_ROWS = 16;
-constexpr int HALO_ROWS = TILE_ROWS + 2;
-constexpr int CB = 64;                 // channels per K block = one 128-byte swizzled row
-constexpr int MAX_WST = 12;
-constexpr int MAX_HST = 4;             // halo ring depth: 2 when the input is L2-resident, up to 4 when it streams from HBM
-constexpr int NUM_EPI_WARPS = 8;       // two warps per TMEM lane quarter, each taking half of the output channels
+constexpr int NUM_EPI_WARPS = 8;      // two warps per TMEM lane quarter, each taking half of the output channels
 constexpr int NUM_THREADS = 64 + 32 * NUM_EPI_WARPS + 32;   // + the output-store warp (staged epilogue)
 constexpr int STORE_WARP = 2 + NUM_EPI_WARPS;
 
@@ -50,8 +43,8 @@ struct TcParams {
   int mode, act, out_f32_c;
   float post_scale, post_shift;
   int nblk, WST, TPS, KS;              // Cin/64, weight ring stages, taps per weight slab (1 or 3), K-split chains
-  int HST, CS, mcast, num_tiles;       // halo stages, cluster size, resident+multicast weights, real tile count
-  uint32_t copy_bytes, halo_stage_bytes, w_slab_bytes, tmem_cols;
+  int HST, mcast, num_tiles;           // halo stages, resident weights, real tile count
+  uint32_t halo_stage_bytes, w_slab_bytes, tmem_cols;
   int tma_out, tma_res;                // staged epilogue: bf16 output / residual tiles through swizzled smem + TMA (see conv_tc_sw.cu)
   const uint8_t* wpk;
   const float* bias;
@@ -72,8 +65,7 @@ using namespace tcptx;   // mbarrier / TMA / tcgen05 wrappers and the UMMA descr
 // Persistent and pipelined: a CTA walks tiles c, c+G, c+2G, ... of its Cout split.  The halo ring (HST stages), the
 // weight ring (or the resident layer, loaded once) and AS TMEM accumulator stages let the TMA producer, the MMA
 // issuer and the epilogue warps work on three different tiles at the same time.
-// H1: single halo box per block, horizontal taps as 128-byte descriptor start offsets (see conv_tc_sw.cu)
-template <int MODE, int TPS, int J, int KS, int H1>
+template <int MODE, int TPS, int J, int KS>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_y,
                   const __grid_constant__ CUtensorMap tmap_r, const TcParams p) {
@@ -81,7 +73,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  uint8_t* halo_base = smem;                                             // HST stages x 3 kx-copies
+  uint8_t* halo_base = smem;                                             // HST halo stages
   uint8_t* w_base = smem + (size_t)p.HST * p.halo_stage_bytes;           // WST weight slabs
   uint64_t* bars = reinterpret_cast<uint64_t*>(w_base + (size_t)p.WST * p.w_slab_bytes);
   uint64_t* halo_full = bars;                    // [MAX_HST]
@@ -103,7 +95,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
 
   // work assignment: grid = nsplit x G CTAs; CTA c of a split owns tiles c, c+G, ...
   const int c_in_split = blockIdx.x % p.G;
-  const int n0 = (blockIdx.x / p.G) * p.Ncta;   // first output channel of this CTA (all CTAs of a cluster share it)
+  const int n0 = (blockIdx.x / p.G) * p.Ncta;   // first output channel of this CTA
   const int my_tiles = c_in_split < p.num_tiles ? (p.num_tiles - c_in_split + p.G - 1) / p.G : 0;
   long long* dbg = p.dbg ? p.dbg + (size_t)blockIdx.x * 64 : nullptr;   // [0,32) phase stamps, [32,64) per-tile stamps
 #define STAMP(i) do { if (dbg) dbg[i] = clock64(); } while (0)
@@ -140,8 +132,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tcgen05_fence_before();
-  if (p.CS > 1) cluster_sync_all();   // every CTA's mbarriers are initialised before any multicast may signal them
-  else __syncthreads();
+  __syncthreads();
   tcgen05_fence_after();
   pdl_launch_dependents();
   const uint32_t tmem_base = *tmem_slot;
@@ -154,9 +145,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   // yields 8J-2 output columns.  Why: an MMA costs ~60 clk whatever N is (the 4 KB A tile read bounds it), so the 64->3
   // output stage at HR resolution used to cost as much per pixel as a 64->64 layer; this needs 12 MMAs per sub-tile, not 36.
   constexpr int nacc = MODE == 1 ? 4 : (MODE == 2 ? 3 : 1);
-  constexpr int ncopies = H1 ? 1 : (MODE == 1 ? 2 : 3);   // horizontal tap offsets that occur (tconv only reads x-1, x)
   constexpr int slabs_per_blk = 9 / TPS;
-  constexpr int row_bytes = ((H1 && MODE != 2) ? 8 * J + 2 : 8 * J) * 128;   // one box row (pixels x 128 B)
+  constexpr int row_bytes = (MODE != 2 ? 8 * J + 2 : 8 * J) * 128;           // one box row (pixels x 128 B)
   constexpr int tile_w = MODE == 2 ? 8 * J - 2 : 8 * J;                      // output columns per tile
   constexpr uint32_t copy_bytes = (uint32_t)(HALO_ROWS * row_bytes);
   const int slabs_per_tile = slabs_per_blk * p.nblk;
@@ -175,24 +165,9 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   if (warp == 0) {
     // ===================== TMA producer =====================
     // Issue cost of one bulk/tensor copy is a few hundred cycles, so independent copies are issued by different lanes.
-    if (p.mcast) {
-      // Resident weights (whole layer fits): they do not depend on the previous layer -> fetch them once, before the
-      // dependency wait.  With CS > 1 each CTA of the cluster fetches 1/CS of every slab and multicasts it.
-      const int sidx = lane;
-      if (sidx < slabs_per_tile) {
-        const uint32_t crank = p.CS > 1 ? cluster_ctarank() : 0;
-        const uint32_t part = p.w_slab_bytes / (uint32_t)p.CS;
-        const uint16_t mask = (uint16_t)((1u << p.CS) - 1u);
-        const int b = sidx / slabs_per_blk, g = sidx - slabs_per_blk * b;
-        mbar_expect_tx(smem_u32(&w_full[sidx]), p.w_slab_bytes);
-        // global layout [blk][tap][cout][64]: a slab = TPS consecutive taps of one block (TPS == 3 only when nsplit == 1)
-        const uint8_t* src = p.wpk + ((size_t)(b * 9 + g * TPS) * p.Cout + n0) * 128 + (size_t)crank * part;
-        const uint32_t dst = smem_u32(w_base + (size_t)sidx * p.w_slab_bytes) + crank * part;
-        if (p.CS > 1) bulk_load_1d_mcast(dst, src, part, smem_u32(&w_full[sidx]), mask);
-        else bulk_load_1d(dst, src, part, smem_u32(&w_full[sidx]));
-      }
-      __syncwarp();
-    }
+    // Resident weights (whole layer fits): they do not depend on the previous layer -> fetch them once, before the
+    // dependency wait.
+    if (p.mcast) fetch_resident_weights<TPS>(lane, slabs_per_tile, p.wpk, p.Cout, n0, p.w_slab_bytes, w_base, w_full, 1);
     // Ring mode: slab sequence q = 0 .. my_tiles*slabs_per_tile-1 through WST stages; the first WST do not depend on
     // the previous layer either -> issue them before the wait.
     const int total_slabs = my_tiles * slabs_per_tile;
@@ -218,12 +193,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
       for (int b = 0; b < p.nblk; ++b) {
         if (lane == 0) {
           mbar_wait(smem_u32(&halo_empty[hs]), hph ^ 1);
-          mbar_expect_tx(smem_u32(&halo_full[hs]), copy_bytes * ncopies);
+          mbar_expect_tx(smem_u32(&halo_full[hs]), copy_bytes);
         }
         __syncwarp();
-        if (lane < ncopies)
-          tma_load_4d(smem_u32(halo_base + (size_t)hs * p.halo_stage_bytes + (size_t)lane * copy_bytes), &tmap,
-                      smem_u32(&halo_full[hs]), b * CB, x0 - 1 + lane, y0 - 1, n);
+        if (lane == 0)
+          tma_load_4d(smem_u32(halo_base + (size_t)hs * p.halo_stage_bytes), &tmap, smem_u32(&halo_full[hs]), b * CB, x0 - 1, y0 - 1, n);
         if (!p.mcast && lane == 0)   // slabs up to the end of this block that are not in flight yet
           for (; next_slab < it * slabs_per_tile + (b + 1) * slabs_per_blk; ++next_slab) issue_slab(next_slab);
         __syncwarp();
@@ -239,10 +213,6 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
         if (lane < J)
           tma_load_4d(smem_u32(stage_base + (size_t)(sg * J + lane) * 16384), &tmap_r, smem_u32(&res_full[sg]), n0, x0 + 8 * lane, y0, n);
       }
-    }
-    if (my_tiles == 0 && p.mcast && lane == 0) {
-      // padding CTA of a cluster: it only relays its share of the weights; stay until they have landed here too
-      for (int sidx = 0; sidx < slabs_per_tile; ++sidx) mbar_wait(smem_u32(&w_full[sidx]), 0);
     }
     __syncwarp();
   } else if (warp == 1) {
@@ -302,15 +272,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
               const int t = g * TPS + tt;
               const int ky = (TPS == 3) ? g : t / 3, kx = (TPS == 3) ? tt : t - 3 * (t / 3);
               int ry, rx, phase;
-              if (MODE == 1) {  // transposed conv: tap -> (input offset, output phase)
-                ry = (ky == 2) ? 0 : 1;
-                rx = (kx == 2) ? 0 : 1;
-                phase = ((ky == 1) ? 2 : 0) + ((kx == 1) ? 1 : 0);
-              } else {
-                ry = ky; rx = kx; phase = 0;
-              }
-              a_off16[tt] = H1 ? ((uint32_t)(rx * 128 + ry * row_bytes)) >> 4
-                               : ((uint32_t)rx * copy_bytes + (uint32_t)(ry * row_bytes)) >> 4;
+              tap_route<MODE>(ky, kx, ry, rx, phase);
+              a_off16[tt] = ((uint32_t)(rx * 128 + ry * row_bytes)) >> 4;
               acc_idx[tt] = (uint32_t)(phase * KS);   // first chain of this tap's accumulator
             }
             // K-split chain of an MMA: KS == 3 -> the tap within the slab (kx), KS == 2 -> parity of the k-step.
@@ -475,28 +438,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
                 if (p.res) {
                   const uint4* rp = reinterpret_cast<const uint4*>(p.res + pix * p.Cout + n0 + c0);
 #pragma unroll
-                  for (int k = 0; k < EW / 8; ++k) {
-                    const uint4 rr = rp[k];
-                    const uint32_t rw[4] = {rr.x, rr.y, rr.z, rr.w};
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                      float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&rw[i]));
-                      v[8 * k + 2 * i] += f.x;
-                      v[8 * k + 2 * i + 1] += f.y;
-                    }
-                  }
+                  for (int k = 0; k < EW / 8; ++k) add_bf16x8(v + 8 * k, rp[k]);
                 }
                 uint4* yp = reinterpret_cast<uint4*>(p.y + pix * p.Cout + n0 + c0);
 #pragma unroll
-                for (int k = 0; k < EW / 8; ++k) {
-                  uint32_t o[4];
-#pragma unroll
-                  for (int i = 0; i < 4; ++i) {
-                    __nv_bfloat162 h = __floats2bfloat162_rn(v[8 * k + 2 * i], v[8 * k + 2 * i + 1]);
-                    o[i] = *reinterpret_cast<uint32_t*>(&h);
-                  }
-                  yp[k] = make_uint4(o[0], o[1], o[2], o[3]);
-                }
+                for (int k = 0; k < EW / 8; ++k) yp[k] = pack_bf16x8(v + 8 * k);
               }
               if (threadIdx.x == 64 && it == 0 && j == 0 && ph == 0) STAMP(12 + ((c0 / EW) & 3));
             }
@@ -533,23 +479,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
           uint4* cell = reinterpret_cast<uint4*>(row + ((((uint32_t)(4 * chalf + k)) ^ sw) << 4));   // XOR swizzle of the TMA box
-          if (p.tma_res) {
-            const uint4 rr = *cell;
-            const uint32_t rw[4] = {rr.x, rr.y, rr.z, rr.w};
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&rw[i]));
-              v[8 * k + 2 * i] += f.x;
-              v[8 * k + 2 * i + 1] += f.y;
-            }
-          }
-          uint32_t o[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            __nv_bfloat162 h = __floats2bfloat162_rn(v[8 * k + 2 * i], v[8 * k + 2 * i + 1]);
-            o[i] = *reinterpret_cast<uint32_t*>(&h);
-          }
-          *cell = make_uint4(o[0], o[1], o[2], o[3]);
+          if (p.tma_res) add_bf16x8(v + 8 * k, *cell);
+          *cell = pack_bf16x8(v + 8 * k);
         }
       };
       for (int it = 0; it < my_tiles; ++it) {
@@ -737,27 +668,9 @@ __global__ void pack_conv3x3_kernel(const float* __restrict__ w, int cin, int co
   }
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
-  return fn;
-}
-
 }  // namespace
 
 long long* teco_g_dbg_timing = nullptr;   // shared with conv_tc_sw.cu
-int teco_conv3x3_tc_one_tile(const teco_tc_desc* d, const void* x, const void* wpk, const float* bias, const void* res,
-                             void* y, const float* res_f32, float* out_f32, void* stream);   // conv_tc_sw.cu
 
 extern "C" int teco_debug_timing(void* buf) {
   teco_g_dbg_timing = (long long*)buf;
@@ -795,225 +708,34 @@ extern "C" int teco_conv3x3_tc(const teco_tc_desc* d, const void* x, const void*
   TECO_CHECK_ARG((((uintptr_t)x) & 15) == 0 && (((uintptr_t)wpk) & 15) == 0 && (((uintptr_t)y) & 15) == 0 &&
                      (((uintptr_t)res) & 15) == 0,
                  "teco_conv3x3_tc: tensors must be 16-byte aligned");
+  TcPlan pl;
+  if (int e = tc_plan(d, y != nullptr, res != nullptr, out_f32 != nullptr, teco_sm_count(), pl)) return e;
+  if (pl.onetile) return teco_conv3x3_tc_onetile(pl, d, x, wpk, bias, res, y, res_f32, out_f32, stream);
 
   TcParams p;
   p.N = d->N; p.H = d->H; p.W = d->W; p.Cin = d->Cin; p.Cout = d->Cout;
+  p.Ncta = pl.Ncta; p.nsplit = pl.nsplit; p.G = pl.G; p.AS = pl.AS;
+  p.tiles_x = pl.tiles_x; p.tiles_y = pl.tiles_y; p.J = pl.J;
   p.mode = d->mode; p.act = d->act; p.out_f32_c = d->out_f32_c;
   p.post_scale = d->post_scale; p.post_shift = d->post_shift;
+  p.nblk = pl.nblk; p.WST = pl.WST; p.TPS = pl.TPS; p.KS = pl.KS;
+  p.HST = pl.HST; p.mcast = pl.mcast; p.num_tiles = pl.num_tiles;
+  p.halo_stage_bytes = pl.halo_stage_bytes; p.w_slab_bytes = pl.w_slab_bytes; p.tmem_cols = pl.tmem_cols;
+  p.tma_out = pl.tma_out; p.tma_res = pl.tma_res;
   p.wpk = (const uint8_t*)wpk; p.bias = bias; p.res = (const __nv_bfloat16*)res; p.y = (__nv_bfloat16*)y;
   p.res_f32 = res_f32; p.out_f32 = out_f32; p.dbg = teco_g_dbg_timing;
-  p.nblk = d->Cin / CB;
-  const int sms = teco_sm_count();
-  const int nacc = d->mode == 1 ? 4 : 1;
-  const size_t budget = 208 * 1024;
-  // few spatial tiles but many output channels (FNet's 16x16 / 32x32 layers): split Cout over CTAs, 64 channels each
-  const long long tiles1 = (long long)d->N * teco_ceil_div(d->H, TILE_ROWS) * teco_ceil_div(d->W, 8);
-  p.nsplit = (d->Cout >= 128 && d->Cout % 64 == 0 && tiles1 * (d->Cout / 64) <= 2LL * sms) ? d->Cout / 64 : 1;
-  if (d->Cout / p.nsplit > 256) p.nsplit = d->Cout / 256;   // VGG's 512-channel layers: N <= 256 per UMMA / TMEM stage
-  p.Ncta = d->Cout / p.nsplit;
-  TECO_CHECK_ARG(nacc * p.Ncta <= 512, "teco_conv3x3_tc: Cout=%d too large for mode %d (TMEM has 512 columns)", d->Cout, d->mode);
-  const size_t tap_bytes = (size_t)p.Ncta * 128;
-  constexpr int H1 = 1;   // single halo box per block, horizontal taps as 128-byte descriptor offsets (the three-box variant lost the A/B and is gone)
-  // bytes of one J = 1 halo stage: one 10-pixel-wide box (23 KB, padded to the swizzle atom) or three 8-pixel boxes
-  const size_t stage1 = H1 ? (((size_t)HALO_ROWS * 10 * 128 + 1023) & ~(size_t)1023) : 3 * (size_t)HALO_ROWS * 8 * 128;
-  const bool single_wave = tiles1 * p.nsplit <= (long long)sms;
-  // Dispatch (same-box A/B, profiles/conv_tc_r01_notes.md): the one-tile-per-CTA kernel is faster for single-wave
-  // launches and for the epilogue-heavy transposed conv (two CTAs per SM); this persistent kernel wins multi-wave convs.
-  // ... except large transposed convs (many waves): persistent CTAs with one staging tile per output phase
-  constexpr int env_tma = 1;   // staged (TMA-store) epilogue wherever the layer qualifies
-  static const int env_tp = [] { const char* e = getenv("TECO_TC_TCONV_PERSIST"); return e ? atoi(e) : 1; }();
-  const bool tconv_persist = env_tp && env_tma && d->mode == 1 && tiles1 >= 4LL * sms && p.nsplit == 1 && p.Ncta == 64 && y && !out_f32 &&
-                             !res && d->H % TILE_ROWS == 0 && d->W % 8 == 0 && d->act < TECO_ACT_TANH24 && p.nblk == 1;
-  if (single_wave || (d->mode == 1 && !tconv_persist))
-    return teco_conv3x3_tc_one_tile(d, x, wpk, bias, res, y, res_f32, out_f32, stream);
-
-  // ---- configuration: (J, HST, weight staging, K-split, accumulator stages, grid)
-  int J = 1;
-  p.mcast = 0; p.CS = 1; p.AS = 1;
-  if (single_wave) {
-    // One tile per CTA, one CTA per SM (e.g. the 128x128 trunk: 128 tiles).  Whole layer resident when it fits: fetched
-    // before the dependency wait and multicast over a 4-CTA cluster (measured 6.2 us vs 6.9 us for a ring, 64->64).
-    p.HST = p.nblk > 1 ? 2 : 1;
-    const size_t a_total1 = (size_t)p.HST * stage1;
-    if (p.nsplit == 1 && a_total1 + 9 * tap_bytes * p.nblk <= budget && 3 * p.nblk <= MAX_WST) {
-      p.mcast = 1; p.TPS = 3; p.WST = 3 * p.nblk;
-      p.CS = tiles1 >= 8 ? 4 : 1;
-    } else if (p.nsplit == 1 && a_total1 + 2 * 3 * tap_bytes <= budget) {
-      p.TPS = 3; p.WST = (int)((budget - a_total1) / (3 * tap_bytes));
-      if (p.WST > 3 * p.nblk) p.WST = 3 * p.nblk;
-      if (p.WST > MAX_WST) p.WST = MAX_WST;
-    } else {
-      p.TPS = 1;
-      int wst = (int)((budget - a_total1) / tap_bytes);
-      if (wst > 9 * p.nblk) wst = 9 * p.nblk;
-      if (wst > MAX_WST) wst = MAX_WST;
-      TECO_CHECK_ARG(wst >= 2, "teco_conv3x3_tc: shared memory budget too small (Cin=%d Cout=%d)", d->Cin, d->Cout);
-      p.WST = wst;
-    }
-  } else {
-    // Multi-wave problems: persistent CTAs (one per SM) walking tiles, double-buffered halo stages and -- when TMEM
-    // allows -- two accumulator stages, so TMA, MMA and epilogue overlap across tiles; the layer's weights stay resident
-    // in shared memory for the whole launch when they fit next to two halo stages.
-    p.HST = 2;
-    const size_t a_total1 = 2 * stage1;
-    if (a_total1 + 9 * tap_bytes * p.nblk <= budget && 3 * p.nblk <= MAX_WST) {
-      p.mcast = 1; p.TPS = 3; p.WST = 3 * p.nblk;             // resident, loaded once per CTA (no cluster: CS = 1)
-    } else if (a_total1 + 2 * 3 * tap_bytes <= budget) {
-      p.TPS = 3; p.WST = (int)((budget - a_total1) / (3 * tap_bytes));
-      if (p.WST > MAX_WST) p.WST = MAX_WST;
-    } else {
-      p.TPS = 1;
-      int wst = (int)((budget - a_total1) / tap_bytes);
-      if (wst > MAX_WST) wst = MAX_WST;
-      TECO_CHECK_ARG(wst >= 2, "teco_conv3x3_tc: shared memory budget too small (Cin=%d Cout=%d)", d->Cin, d->Cout);
-      p.WST = wst;
-    }
-  }
-  // Multi-wave 3x3 convs with <= 64 output channels per CTA: two 16x8 sub-tiles per tile and two K-split chains each
-  // (4 independent accumulators) instead of one sub-tile with three -- a third less TMEM read traffic in the epilogue
-  // (the 64 B/clk tcgen05.ld path bounds it) and a 16+2 pixel wide halo row instead of two 8+2 ones.
-  static const int env_j2 = [] { const char* e = getenv("TECO_TC_J2"); return e ? atoi(e) : 1; }();
-  int ks_force = 0;
-  if (!single_wave && H1 && env_j2 && d->mode == 0 && p.TPS == 3 && p.mcast && p.Ncta <= 64 &&
-      tiles1 >= 4LL * sms) {
-    const size_t stage2 = ((size_t)HALO_ROWS * 18 * 128 + 1023) & ~(size_t)1023;
-    if (2 * stage2 + 9 * tap_bytes * p.nblk <= budget) { J = 2; ks_force = 2; }
-  }
-  // Narrow fp32 output stage (generator 64->3, fnet 32->2) on many tiles: the kx-fused kernel (MODE 2 above)
-  static const int env_kx = [] { const char* e = getenv("TECO_TC_KX"); return e ? atoi(e) : 1; }();
-  const bool kx = env_kx && H1 && !single_wave && d->mode == 0 && out_f32 && !y && !res && d->Cout == 16 && p.nsplit == 1 && p.nblk == 1 &&
-                  d->out_f32_c <= 4 && p.mcast && p.TPS == 3;
-  if (kx) {
-    double best = 0.0;
-    for (int jj = 2; jj <= 4; ++jj) {   // widest use of the 8*jj halo columns: W / (tiles * 8 jj)
-      const double eff = (double)d->W / ((double)teco_ceil_div(d->W, 8 * jj - 2) * 8 * jj);
-      if (eff > best + 1e-9) { best = eff; J = jj; }
-    }
-    ks_force = 1;
-  }
-  const int box_w = (H1 && !kx) ? 8 * J + 2 : 8 * J;
-  p.J = J;
-  p.tiles_x = kx ? teco_ceil_div(d->W, 8 * J - 2) : teco_ceil_div(d->W, 8 * J);
-  p.tiles_y = teco_ceil_div(d->H, TILE_ROWS);
-  p.num_tiles = (int)((long long)d->N * p.tiles_x * p.tiles_y);
-  p.copy_bytes = (uint32_t)(HALO_ROWS * box_w * 128);
-  p.halo_stage_bytes = H1 ? ((p.copy_bytes + 1023u) & ~1023u) : 3 * p.copy_bytes;
-  // Input larger than ~half of L2 streams from HBM: one tile of look-ahead (HST = 2) leaves the CTA waiting on DRAM
-  // latency (the 64->16 output stage at 296 x 128x128 ran 6300 clk per tile against ~2900 of work); use the shared memory
-  // the configuration leaves free for a deeper ring.
-  const bool tma_possible = tconv_persist || (env_tma && d->mode == 0 && y && !out_f32 && p.Ncta == 64 && d->act < TECO_ACT_TANH24);
-  const size_t staging_bytes = tconv_persist ? 1024 + (size_t)4 * 16384 : 1024 + (size_t)2 * J * 16384;
-  const double in_bytes = (double)d->N * d->H * d->W * d->Cin * 2.0;
-  if (!single_wave && p.nblk == 1 && in_bytes > 48e6) {
-    const size_t fixed = (size_t)p.WST * p.TPS * tap_bytes + (tma_possible ? staging_bytes : 0) + 8192;
-    while (p.HST < MAX_HST && fixed + (size_t)(p.HST + 1) * p.halo_stage_bytes <= 232448 - 2048) ++p.HST;
-  }
-  const size_t a_total = (size_t)p.HST * p.halo_stage_bytes;
-  p.w_slab_bytes = (uint32_t)(p.TPS * tap_bytes);
-  p.KS = ks_force ? ks_force : ((p.TPS == 3 && d->mode == 0 && J * 3 * p.Ncta <= 512) ? 3 : 1);
-  const uint32_t stage_cols = (uint32_t)(J * (kx ? 3 : nacc) * p.KS * p.Ncta);
-  if (!single_wave && 2 * stage_cols <= 512) p.AS = 2;
-  uint32_t cols = stage_cols * (uint32_t)p.AS, tc = 32;
-  while (tc < cols) tc <<= 1;
-  p.tmem_cols = tc;
-  if (single_wave) p.G = (p.num_tiles + p.CS - 1) / p.CS * p.CS;   // padded to the cluster size
-  else p.G = p.num_tiles < sms ? p.num_tiles : sms;
-  p.tma_out = tma_possible ? 1 : 0;
-  p.tma_res = (p.tma_out && res) ? 1 : 0;
-  size_t smem_bytes = 1024 + a_total + (size_t)p.WST * p.w_slab_bytes + (2 * MAX_HST + 2 * MAX_WST + 4 + 1) * 8 + 256 * sizeof(float) + 128 +
-                      (p.tma_out ? staging_bytes : 0);
-  if (smem_bytes > 232448 && p.tma_out) {       // 227 KB: the opt-in maximum of dynamic shared memory per block on sm_100
-    TECO_CHECK_ARG(!tconv_persist, "teco_conv3x3_tc: persistent transposed conv does not fit in shared memory");
-    smem_bytes -= staging_bytes;
-    p.tma_out = p.tma_res = 0;
-  }
-
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) {
-    teco_set_error("teco_conv3x3_tc: cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
-    return TECO_E_CUDA;
-  }
-  CUtensorMap tmap;
-  const cuuint64_t gdim[4] = {(cuuint64_t)d->Cin, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-  const cuuint64_t gstr[3] = {(cuuint64_t)d->Cin * 2, (cuuint64_t)d->W * d->Cin * 2, (cuuint64_t)d->H * d->W * d->Cin * 2};
-  const cuuint32_t box[4] = {(cuuint32_t)CB, (cuuint32_t)box_w, (cuuint32_t)HALO_ROWS, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), gdim, gstr, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) {
-    teco_set_error("teco_conv3x3_tc: cuTensorMapEncodeTiled failed with CUresult %d (N=%d H=%d W=%d Cin=%d)", (int)cr, d->N,
-                   d->H, d->W, d->Cin);
-    return TECO_E_CUDA;
-  }
-  CUtensorMap tmap_y = tmap, tmap_r = tmap;   // placeholders when the staged epilogue is off
-  if (p.tma_out && d->mode == 1) {
-    // output [N, 2H, 2W, C] as {C, px, x, py, n*H + y}: one box = the 16x8 pixels of one sub-pixel phase (H % 16 == 0, so a
-    // box never runs from one image into the next)
-    const cuuint64_t odim[5] = {(cuuint64_t)d->Cout, 2, (cuuint64_t)d->W, 2, (cuuint64_t)d->N * d->H};
-    const cuuint64_t ostr[4] = {(cuuint64_t)d->Cout * 2, (cuuint64_t)d->Cout * 4, (cuuint64_t)d->W * d->Cout * 4,
-                                (cuuint64_t)d->W * d->Cout * 8};
-    const cuuint32_t obox[5] = {64, 1, 8, 1, (cuuint32_t)TILE_ROWS};
-    const cuuint32_t estr5[5] = {1, 1, 1, 1, 1};
-    cr = enc(&tmap_y, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, y, odim, ostr, obox, estr5, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) {
-      teco_set_error("teco_conv3x3_tc: cuTensorMapEncodeTiled (transposed-conv output) failed with CUresult %d", (int)cr);
-      return TECO_E_CUDA;
-    }
-  } else if (p.tma_out) {
-    const cuuint64_t odim[4] = {(cuuint64_t)d->Cout, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    const cuuint64_t ostr[3] = {(cuuint64_t)d->Cout * 2, (cuuint64_t)d->W * d->Cout * 2, (cuuint64_t)d->H * d->W * d->Cout * 2};
-    const cuuint32_t obox[4] = {64, 8, (cuuint32_t)TILE_ROWS, 1};
-    cr = enc(&tmap_y, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, odim, ostr, obox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr == CUDA_SUCCESS && p.tma_res)
-      cr = enc(&tmap_r, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(res), odim, ostr, obox, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) {
-      teco_set_error("teco_conv3x3_tc: cuTensorMapEncodeTiled (output tile) failed with CUresult %d", (int)cr);
-      return TECO_E_CUDA;
-    }
-  }
-  using KernelT = void (*)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const TcParams);
-  KernelT kern = nullptr;
-#define TECO_PICK(M, T, JJ, K)                                              \
-  if ((kx ? 2 : d->mode) == M && p.TPS == T && J == JJ && p.KS == K)        \
-    kern = conv3x3_tc_kernel<M, T, JJ, K, 1>;
-  TECO_PICK(0, 3, 2, 2) TECO_PICK(0, 3, 1, 3) TECO_PICK(0, 3, 2, 3) TECO_PICK(0, 3, 1, 1) TECO_PICK(0, 3, 2, 1) TECO_PICK(0, 1, 1, 1) TECO_PICK(0, 1, 2, 1)
-  TECO_PICK(1, 3, 1, 1) TECO_PICK(1, 3, 2, 1) TECO_PICK(1, 1, 1, 1) TECO_PICK(1, 1, 2, 1)
+  CUtensorMap maps[3];
+  if (int e = tc_encode_maps(pl, d, x, y, res, maps)) return e;
+  void (*kern)(CUtensorMap, CUtensorMap, CUtensorMap, TcParams) = nullptr;
+#define TECO_PICK(M, T, JJ, K) \
+  if (pl.kmode == M && pl.TPS == T && pl.J == JJ && pl.KS == K) kern = conv3x3_tc_kernel<M, T, JJ, K>;
+  TECO_PICK(0, 3, 2, 2) TECO_PICK(0, 3, 1, 3) TECO_PICK(0, 3, 1, 1) TECO_PICK(0, 1, 1, 1)
+  TECO_PICK(1, 3, 1, 1)
   TECO_PICK(2, 3, 2, 1) TECO_PICK(2, 3, 3, 1) TECO_PICK(2, 3, 4, 1)
 #undef TECO_PICK
   if (!kern) {
-    teco_set_error("teco_conv3x3_tc: no kernel instantiation for mode=%d TPS=%d J=%d KS=%d", d->mode, p.TPS, J, p.KS);
+    teco_set_error("teco_conv3x3_tc: no kernel instantiation for mode=%d TPS=%d J=%d KS=%d", pl.kmode, pl.TPS, pl.J, pl.KS);
     return TECO_E_UNSUPPORTED;
   }
-  TECO_CUDA_CALL(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-  const unsigned ctas = (unsigned)(p.G * p.nsplit);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(ctas);
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = smem_bytes;
-  cfg.stream = (cudaStream_t)stream;
-  cudaLaunchAttribute attrs[2];
-  int na = 0;
-  attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // PDL: prologue overlaps the previous kernel's tail
-  attrs[na].val.programmaticStreamSerializationAllowed = 1;
-  ++na;
-  if (p.CS > 1) {
-    attrs[na].id = cudaLaunchAttributeClusterDimension;
-    attrs[na].val.clusterDim.x = (unsigned)p.CS;
-    attrs[na].val.clusterDim.y = 1;
-    attrs[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = attrs;
-  cfg.numAttrs = na;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, kern, tmap, tmap_y, tmap_r, p);
-  if (le != cudaSuccess) {
-    teco_set_error("teco_conv3x3_tc: launch failed: %s (grid %u, cluster %d, smem %zu)", cudaGetErrorString(le), ctas, p.CS, smem_bytes);
-    return TECO_E_CUDA;
-  }
-  return TECO_OK;
+  return tc_launch(kern, (int)TC_SMEM_MAX, NUM_THREADS, pl, maps, p, stream);
 }

@@ -1,46 +1,15 @@
-// ONE-TILE-PER-CTA variant of the tcgen05 convolution (see conv_tc.cu for the design notes and the persistent variant).
-// Used for single-wave launches (tiles <= SMs, e.g. the 128x128 generator trunk) and for the transposed convolutions:
+// ONE-TILE-PER-CTA variant of the tcgen05 convolution (see conv_tc.cu for the design notes and the persistent variant;
+// tc_plan in conv_tc_common.cuh picks between them).
+// Used for single-wave launches (tiles <= SMs, e.g. the 128x128 generator trunk) and for most transposed convolutions:
 // same-box A/B (profiles/conv_tc_r01_notes.md) showed this variant 1.3 us faster per single-wave layer and its
 // two-CTAs-per-SM ring faster on the epilogue-heavy transposed conv, while the persistent kernel wins every multi-wave conv.
-// bf16 3x3 convolution / 3x3-stride-2 transposed convolution on the 5th-gen tensor cores (sm_100a):
-// TMA halo tiles -> shared memory -> tcgen05.mma (kind::f16, fp32 accumulators in TMEM) -> tcgen05.ld
-// epilogue (bias, activation, residual, bf16 store; or fp32 "+bicubic, *2-1" output stage).
-//
-// Replaces, layer by layer, the cuDNN convolutions behind conv2()/conv2_tran() of the reference
-// (lib/ops.py:35-56) as used by generator_F (lib/frvsr.py:44-88) and fnet (lib/frvsr.py:4-41).
-//
-// Implicit GEMM, no im2col buffer:
-//   CTA tile  = 16 image rows x (8*J) pixels; every 16x8 sub-tile is one UMMA accumulator with M = 128.
-//   A operand = NHWC bf16 activations, 64 channels = one 128-byte row per pixel.  Per 64-channel block the halo is
-//               staged by THREE 4-D TMA boxes (64 ch, 8J px, 18 rows, 1 image), one per horizontal tap offset kx,
-//               with SWIZZLE_128B.  Each box is the UMMA canonical K-major SW128 layout as it lands
-//               (8 consecutive pixels = one 1024-byte swizzle atom, SBO = one box row).  Vertical taps ky are
-//               descriptor start-address offsets of whole box rows (atom aligned), so 3 loads serve 9 taps.
-//               TMA out-of-bounds zero fill implements TF 'SAME' padding.
-//   B operand = weights pre-packed on the device as [cin/64][tap][cout][64 cin] bf16 in the same SW128 image,
-//               streamed by 1-D bulk copies.  When a whole layer fits (64->64: 72 KB) the slabs are fetched once,
-//               BEFORE the programmatic-dependent-launch wait, and multicast across a 4-CTA cluster.
-//   D         = fp32 in TMEM, column block (sub-tile, phase) * Cout.
-// Transposed conv (stride 2, TF 'SAME', y[i] = sum_j x[j] w[i-2j]) is the same loop with the nine taps routed to
-// four sub-pixel phase accumulators (SURVEY.md A.3) and a 2x interleaving epilogue.
-//
-// Why SW128 and not the no-swizzle layout (round-1 measurement, profiles/conv_tc_r01_notes.md): with 16-byte core
-// matrix rows every tcgen05.mma took ~250 cycles instead of ~32-48, and the 16-byte TMA rows ran at ~10 B/clk/SM.
-//
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2..9 = epilogue
 // (one epilogue warp per scheduler is latency-bound: ~1000 clk per 32 channels; two per scheduler halve it).
-#include <cuda.h>
-#include <cstdlib>
 #include <type_traits>
-#include "teco_common.cuh"
-#include "tc_ptx.cuh"
+#include "conv_tc_common.cuh"
 
 namespace {
 
-constexpr int TILE_ROWS = 16;
-constexpr int HALO_ROWS = TILE_ROWS + 2;
-constexpr int CB = 64;                 // channels per K block = one 128-byte swizzled row
-constexpr int MAX_WST = 12;
 constexpr int NUM_EPI_WARPS = 8;       // two warps per TMEM lane quarter, each taking half of the output channels
 constexpr int NUM_THREADS = 64 + 32 * NUM_EPI_WARPS;
 
@@ -55,7 +24,7 @@ struct TcParams {
   int late_trigger;                    // trigger the dependent launch after the MMAs instead of after the prologue
   uint32_t stage2_bytes;               // second staging region after the weights: residual tiles (conv) / ping-pong tile (tconv)
   int tma_out, tma_res;                // bf16 output / residual tiles travel through swizzled smem staging + TMA (Ncta == 64, conv)
-  uint32_t copy_bytes, halo_stage_bytes, w_slab_bytes, tmem_cols;
+  uint32_t halo_stage_bytes, w_slab_bytes, tmem_cols;
   const uint8_t* wpk;
   const float* bias;
   const __nv_bfloat16* res;
@@ -71,13 +40,10 @@ using namespace tcptx;   // mbarrier / TMA / tcgen05 wrappers and the UMMA descr
 // MODE 0 conv / 1 transposed conv; TPS taps per weight slab; J sub-tiles per CTA; KS K-split accumulator chains.
 // They are compile-time so that the MMA issue loop is a fully unrolled stream of UTCHMMA whose descriptors differ
 // from per-stage bases by immediates (uniform-datapath adds, no per-instruction R2UR).
-// H1 = 1: ONE halo box (8J+2 pixels wide) per block instead of one box per horizontal tap; the horizontal taps are
-// descriptor start offsets of whole 128-byte pixel rows (not swizzle-atom aligned: the SW128 XOR is a function of the
-// absolute shared-memory address bits, which is also how TMA wrote the box; the descriptor's base-offset field stays 0 --
-// setting it to (addr >> 7) & 7 was tested on the B200 and gives wrong results).  2.4x less L2->smem traffic, 23 KB per stage.
-template <int MODE, int TPS, int J, int KS, int H1>
+// One halo box (8J+2 pixels wide) per block: 2.4x less L2->smem traffic than one box per horizontal tap, 23 KB per stage.
+template <int MODE, int TPS, int J, int KS>
 __global__ void __launch_bounds__(NUM_THREADS, 2)
-conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_y,
+conv3x3_tc_onetile_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_y,
                   const __grid_constant__ CUtensorMap tmap_r, const TcParams p) {
   // SWIZZLE_128B needs 1024-byte aligned tiles; the dynamic window starts on such a boundary (no static shared memory in
   // this kernel) -- relied upon instead of a 1 KB slack so that two trunk-layer CTAs (112.3 KB each) share an SM.
@@ -86,7 +52,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   if ((smem_u32(smem_raw) & 1023u) != 0u) __trap();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
-  uint8_t* halo_base = smem;                                             // HST stages x 3 kx-copies
+  uint8_t* halo_base = smem;                                             // HST halo stages
   uint8_t* w_base = smem + (size_t)p.HST * p.halo_stage_bytes;           // WST weight slabs
   // residual staging tiles (J x 16 KB, TMA box image) follow the weights; the OUTPUT staging tiles reuse the halo
   // stages, which are dead once the accumulators are complete
@@ -152,32 +118,15 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   if (threadIdx.x == 0) STAMP(1);
 
   constexpr int nacc = MODE == 1 ? 4 : 1;
-  constexpr int ncopies = H1 ? 1 : (MODE == 1 ? 2 : 3);   // horizontal tap offsets that occur (tconv only reads x-1, x)
   constexpr int slabs_per_blk = 9 / TPS;
-  constexpr int row_bytes = (H1 ? 8 * J + 2 : 8 * J) * 128;   // one box row (pixels x 128 B)
+  constexpr int row_bytes = (8 * J + 2) * 128;   // one box row (pixels x 128 B)
   constexpr uint32_t copy_bytes = (uint32_t)(HALO_ROWS * row_bytes);
 
   if (warp == 0) {
     // ===================== TMA producer =====================
     // Issue cost of one bulk/tensor copy is a few hundred cycles, so independent copies are issued by different lanes.
-    if (p.mcast) {
-      // Weights do not depend on the previous layer: fetch them before the dependency wait.  Each CTA of the
-      // cluster fetches 1/CS of every slab and multicasts it to all CS CTAs (one L2 read per cluster).
-      const int sidx = lane;
-      if (sidx < slabs_per_blk * p.nblk) {
-        const uint32_t crank = p.CS > 1 ? cluster_ctarank() : 0;
-        const uint32_t part = p.w_slab_bytes / (uint32_t)p.CS;
-        const uint16_t mask = (uint16_t)((1u << p.CS) - 1u);
-        const int b = sidx / slabs_per_blk, g = sidx - slabs_per_blk * b;
-        mbar_expect_tx(smem_u32(&w_full[sidx]), p.w_slab_bytes);
-        // global layout [blk][tap][cout][64]: a slab = TPS consecutive taps of one block (TPS == 3 only when nsplit == 1)
-        const uint8_t* src = p.wpk + ((size_t)(b * 9 + g * TPS) * p.Cout + n0) * 128 + (size_t)crank * part;
-        const uint32_t dst = smem_u32(w_base + (size_t)sidx * p.w_slab_bytes) + crank * part;
-        if (p.CS > 1) bulk_load_1d_mcast(dst, src, part, smem_u32(&w_full[sidx]), mask);
-        else bulk_load_1d(dst, src, part, smem_u32(&w_full[sidx]));
-      }
-      __syncwarp();
-    }
+    // Weights do not depend on the previous layer: fetch them before the dependency wait.
+    if (p.mcast) fetch_resident_weights<TPS>(lane, slabs_per_blk * p.nblk, p.wpk, p.Cout, n0, p.w_slab_bytes, w_base, w_full, p.CS);
     // Ring mode: the first WST weight slabs do not depend on the previous layer either -> issue them before the wait.
     const int total_slabs = slabs_per_blk * p.nblk;
     int next_slab = 0;
@@ -199,12 +148,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
       for (int b = 0; b < p.nblk; ++b) {
         if (lane == 0) {
           mbar_wait(smem_u32(&halo_empty[hs]), hph ^ 1);
-          mbar_expect_tx(smem_u32(&halo_full[hs]), copy_bytes * ncopies);
+          mbar_expect_tx(smem_u32(&halo_full[hs]), copy_bytes);
         }
         __syncwarp();
-        if (lane < ncopies)
-          tma_load_4d(smem_u32(halo_base + (size_t)hs * p.halo_stage_bytes + (size_t)lane * copy_bytes), &tmap,
-                      smem_u32(&halo_full[hs]), b * CB, x0 - 1 + lane, y0 - 1, n);
+        if (lane == 0)
+          tma_load_4d(smem_u32(halo_base + (size_t)hs * p.halo_stage_bytes), &tmap, smem_u32(&halo_full[hs]), b * CB, x0 - 1, y0 - 1, n);
         if (!p.mcast && lane == 0) {
           for (; next_slab < (b + 1) * slabs_per_blk; ++next_slab) {   // slabs of this block not yet in flight
             const int st = next_slab % p.WST, use = next_slab / p.WST;
@@ -258,15 +206,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
             const int t = g * TPS + tt;
             const int ky = (TPS == 3) ? g : t / 3, kx = (TPS == 3) ? tt : t - 3 * (t / 3);
             int ry, rx, phase;
-            if (MODE == 1) {  // transposed conv: tap -> (input offset, output phase)
-              ry = (ky == 2) ? 0 : 1;
-              rx = (kx == 2) ? 0 : 1;
-              phase = ((ky == 1) ? 2 : 0) + ((kx == 1) ? 1 : 0);
-            } else {
-              ry = ky; rx = kx; phase = 0;
-            }
-            a_off16[tt] = H1 ? ((uint32_t)(rx * 128 + ry * row_bytes)) >> 4
-                             : ((uint32_t)rx * copy_bytes + (uint32_t)(ry * row_bytes)) >> 4;
+            tap_route<MODE>(ky, kx, ry, rx, phase);
+            a_off16[tt] = ((uint32_t)(rx * 128 + ry * row_bytes)) >> 4;
             acc_idx[tt] = (uint32_t)(phase * KS + (KS > 1 ? tt : 0));
           }
           const uint32_t started_now = started;
@@ -373,28 +314,13 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
                 mbar_wait_warp(smem_u32(res_full), 0);
                 const uint8_t* rs = stage_res + (size_t)j * 16384 + rowoff;
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const uint4 rr = *reinterpret_cast<const uint4*>(rs + ((((uint32_t)(4 * chalf + k)) ^ ((uint32_t)m & 7u)) << 4));
-                  const uint32_t rw[4] = {rr.x, rr.y, rr.z, rr.w};
-#pragma unroll
-                  for (int i = 0; i < 4; ++i) {
-                    float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&rw[i]));
-                    v[8 * k + 2 * i] += f.x;
-                    v[8 * k + 2 * i + 1] += f.y;
-                  }
-                }
+                for (int k = 0; k < 4; ++k)
+                  add_bf16x8(v + 8 * k, *reinterpret_cast<const uint4*>(rs + ((((uint32_t)(4 * chalf + k)) ^ ((uint32_t)m & 7u)) << 4)));
               }
               uint8_t* os = stage_out + (size_t)j * 16384 + rowoff;
 #pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                uint32_t o[4];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                  __nv_bfloat162 h = __floats2bfloat162_rn(v[8 * k + 2 * i], v[8 * k + 2 * i + 1]);
-                  o[i] = *reinterpret_cast<uint32_t*>(&h);
-                }
-                *reinterpret_cast<uint4*>(os + ((((uint32_t)(4 * chalf + k)) ^ ((uint32_t)m & 7u)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
-              }
+              for (int k = 0; k < 4; ++k)
+                *reinterpret_cast<uint4*>(os + ((((uint32_t)(4 * chalf + k)) ^ ((uint32_t)m & 7u)) << 4)) = pack_bf16x8(v + 8 * k);
               continue;
             }
             if (MODE == 1 && EW == 32 && p.tma_out) {
@@ -408,15 +334,8 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
               }
               uint8_t* os = stg + (uint32_t)m * 128u;
 #pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                uint32_t o[4];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                  __nv_bfloat162 h = __floats2bfloat162_rn(v[8 * k + 2 * i], v[8 * k + 2 * i + 1]);
-                  o[i] = *reinterpret_cast<uint32_t*>(&h);
-                }
-                *reinterpret_cast<uint4*>(os + ((((uint32_t)(4 * chalf + k)) ^ ((uint32_t)m & 7u)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
-              }
+              for (int k = 0; k < 4; ++k)
+                *reinterpret_cast<uint4*>(os + ((((uint32_t)(4 * chalf + k)) ^ ((uint32_t)m & 7u)) << 4)) = pack_bf16x8(v + 8 * k);
               fence_async_smem();
               asm volatile("bar.sync 1, %0;" ::"n"(32 * NUM_EPI_WARPS) : "memory");
               if (threadIdx.x == 64) {
@@ -439,28 +358,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
               if (p.res) {
                 const uint4* rp = reinterpret_cast<const uint4*>(p.res + pix * p.Cout + n0 + c0);
 #pragma unroll
-                for (int k = 0; k < EW / 8; ++k) {
-                  const uint4 rr = rp[k];
-                  const uint32_t rw[4] = {rr.x, rr.y, rr.z, rr.w};
-#pragma unroll
-                  for (int i = 0; i < 4; ++i) {
-                    float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&rw[i]));
-                    v[8 * k + 2 * i] += f.x;
-                    v[8 * k + 2 * i + 1] += f.y;
-                  }
-                }
+                for (int k = 0; k < EW / 8; ++k) add_bf16x8(v + 8 * k, rp[k]);
               }
               uint4* yp = reinterpret_cast<uint4*>(p.y + pix * p.Cout + n0 + c0);
 #pragma unroll
-              for (int k = 0; k < EW / 8; ++k) {
-                uint32_t o[4];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                  __nv_bfloat162 h = __floats2bfloat162_rn(v[8 * k + 2 * i], v[8 * k + 2 * i + 1]);
-                  o[i] = *reinterpret_cast<uint32_t*>(&h);
-                }
-                yp[k] = make_uint4(o[0], o[1], o[2], o[3]);
-              }
+              for (int k = 0; k < EW / 8; ++k) yp[k] = pack_bf16x8(v + 8 * k);
             }
             if (threadIdx.x == 64 && j == 0 && ph == 0) STAMP(12 + ((c0 / EW) & 3));
           }
@@ -493,44 +395,22 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   }
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
-  return fn;
-}
-
 }  // namespace
 
-extern long long* teco_g_dbg_timing;   // set by teco_debug_timing (conv_tc.cu)
-
-int teco_conv3x3_tc_one_tile(const teco_tc_desc* d, const void* x, const void* wpk, const float* bias, const void* res,
-                               void* y, const float* res_f32, float* out_f32, void* stream) {
-  TECO_CHECK_ARG(d && x && wpk, "teco_conv3x3_tc(one-tile): NULL argument");
-  TECO_CHECK_ARG(y || out_f32, "teco_conv3x3_tc(one-tile): no output buffer");
-  TECO_CHECK_ARG(d->N > 0 && d->H > 0 && d->W > 0, "teco_conv3x3_tc(one-tile): bad shape N=%d H=%d W=%d", d->N, d->H, d->W);
-  TECO_CHECK_ARG(d->Cin >= 64 && d->Cin % 64 == 0 && d->Cin <= 512, "teco_conv3x3_tc(one-tile): Cin must be a multiple of 64 in [64,512] (got %d)", d->Cin);
-  TECO_CHECK_ARG(d->Cout >= 16 && d->Cout % 16 == 0 && d->Cout <= 512, "teco_conv3x3_tc(one-tile): Cout must be a multiple of 16 in [16,512] (got %d)", d->Cout);
-  TECO_CHECK_ARG(d->mode == 0 || d->mode == 1, "teco_conv3x3_tc(one-tile): unknown mode %d", d->mode);
-  TECO_CHECK_ARG(d->act >= 0 && d->act <= TECO_ACT_SIGMOID, "teco_conv3x3_tc(one-tile): unknown activation %d", d->act);
-  TECO_CHECK_ARG(!out_f32 || (d->out_f32_c > 0 && d->out_f32_c <= d->Cout), "teco_conv3x3_tc(one-tile): bad out_f32_c");
-  TECO_CHECK_ARG((((uintptr_t)x) & 15) == 0 && (((uintptr_t)wpk) & 15) == 0 && (((uintptr_t)y) & 15) == 0 &&
-                     (((uintptr_t)res) & 15) == 0,
-                 "teco_conv3x3_tc(one-tile): tensors must be 16-byte aligned");
-
+// Launches conv3x3_tc_onetile_kernel as planned by tc_plan; teco_conv3x3_tc (conv_tc.cu) has validated the arguments.
+int teco_conv3x3_tc_onetile(const TcPlan& pl, const teco_tc_desc* d, const void* x, const void* wpk, const float* bias, const void* res,
+                            void* y, const float* res_f32, float* out_f32, void* stream) {
   TcParams p;
   p.N = d->N; p.H = d->H; p.W = d->W; p.Cin = d->Cin; p.Cout = d->Cout;
+  p.Ncta = pl.Ncta; p.nsplit = pl.nsplit; p.tiles_pad = pl.G;
+  p.tiles_x = pl.tiles_x; p.tiles_y = pl.tiles_y; p.J = pl.J;
   p.mode = d->mode; p.act = d->act; p.out_f32_c = d->out_f32_c;
   p.post_scale = d->post_scale; p.post_shift = d->post_shift;
+  p.nblk = pl.nblk; p.WST = pl.WST; p.TPS = pl.TPS; p.KS = pl.KS;
+  p.HST = pl.HST; p.CS = pl.CS; p.mcast = pl.mcast; p.num_tiles = pl.num_tiles;
+  p.late_trigger = pl.late_trigger; p.stage2_bytes = pl.stage2_bytes;
+  p.tma_out = pl.tma_out; p.tma_res = pl.tma_res;
+  p.halo_stage_bytes = pl.halo_stage_bytes; p.w_slab_bytes = pl.w_slab_bytes; p.tmem_cols = pl.tmem_cols;
   p.wpk = (const uint8_t*)wpk; p.bias = bias; p.res = (const __nv_bfloat16*)res; p.y = (__nv_bfloat16*)y;
   p.res_f32 = res_f32; p.out_f32 = out_f32; p.dbg = teco_g_dbg_timing;
   if (p.dbg) {   // consecutive launches stamp consecutive [256][32] slices (tools/bench_conv.py chain)
@@ -540,166 +420,19 @@ int teco_conv3x3_tc_one_tile(const teco_tc_desc* d, const void* x, const void* w
     p.dbg = teco_g_dbg_timing + (size_t)(launch_idx % 8) * 256 * 32;
     ++launch_idx;
   }
-  p.nblk = d->Cin / CB;
-  p.HST = p.nblk > 1 ? 2 : 1;
-  constexpr int H1 = 1;   // single halo box per block, horizontal taps as 128-byte descriptor offsets (the three-box variant lost the A/B and is gone)
-  // few spatial tiles but many output channels (FNet's 16x16 / 32x32 layers): split Cout over CTAs, 64 channels each
-  {
-    long long t1 = (long long)d->N * teco_ceil_div(d->H, TILE_ROWS) * teco_ceil_div(d->W, 8);
-    p.nsplit = (d->Cout >= 128 && d->Cout % 64 == 0 && t1 * (d->Cout / 64) <= 2LL * teco_sm_count()) ? d->Cout / 64 : 1;
-    if (d->Cout / p.nsplit > 256) p.nsplit = d->Cout / 256;
-    p.Ncta = d->Cout / p.nsplit;
-  }
-  const int nacc = d->mode == 1 ? 4 : 1;
-  const size_t budget = 208 * 1024;
-  const int sms = teco_sm_count();
-  // sub-tiles per CTA: prefer the wider tile when it still yields >= 2 waves of CTAs and fits TMEM / smem
-  int J = 1;
-  for (int j = 2; j >= 1; --j) {
-    if (j * nacc * p.Ncta > 512) continue;
-    size_t a_bytes = H1 ? (size_t)p.HST * (((size_t)HALO_ROWS * (8 * j + 2) * 128 + 1023) & ~(size_t)1023)
-                        : (size_t)p.HST * 3 * HALO_ROWS * 8 * j * 128;
-    if (a_bytes + 2 * (size_t)p.Ncta * 128 > budget) continue;
-    long long tiles = (long long)d->N * teco_ceil_div(d->H, TILE_ROWS) * teco_ceil_div(d->W, 8 * j);
-    static const int env_j = [] { const char* e = getenv("TECO_TC_J"); return e ? atoi(e) : 0; }();
-    if (tiles >= 2LL * sms || j == 1 || j == env_j) { J = j; break; }
-  }
-  TECO_CHECK_ARG(J * nacc * p.Ncta <= 512, "teco_conv3x3_tc(one-tile): Cout=%d too large for mode %d (TMEM has 512 columns)", d->Cout, d->mode);
-  p.J = J;
-  p.tiles_x = teco_ceil_div(d->W, 8 * J);
-  p.tiles_y = teco_ceil_div(d->H, TILE_ROWS);
-  p.copy_bytes = (uint32_t)(HALO_ROWS * (H1 ? 8 * J + 2 : 8 * J) * 128);
-  p.halo_stage_bytes = H1 ? ((p.copy_bytes + 1023u) & ~1023u) : 3 * p.copy_bytes;
-  const size_t a_total = (size_t)p.HST * p.halo_stage_bytes;
-  const size_t tap_bytes = (size_t)p.Ncta * 128;
-  // whole layer resident?  then 3 taps per slab (3 barriers per block), fetched once, multicast over a 4-CTA cluster
-  p.num_tiles = (int)((long long)d->N * p.tiles_x * p.tiles_y);
-  // Weight staging.  Preferred: a 2-deep ring of 3-tap slabs -- with the halo copies that is ~105 KB, so TWO CTAs fit per SM
-  // and programmatic dependent launch really overlaps the next layer's prologue + weight prefetch with this layer's
-  // MMA/epilogue.  (A whole resident layer, 128 KB, multicast over a cluster, serialised the layers: round-1 notes.)
-  const size_t half_sm = 112 * 1024;
-  p.mcast = 0;
-  const bool single_wave = (long long)p.num_tiles * p.nsplit <= (long long)sms;
-  if (single_wave && p.nsplit == 1 && a_total + 9 * tap_bytes * p.nblk <= budget && 3 * p.nblk <= MAX_WST) {
-    // one CTA per SM anyway (e.g. the 128x128 trunk: 128 tiles): whole layer resident, fetched before the dependency
-    // wait and multicast over a 4-CTA cluster -- measured 6.2 us vs 6.9 us for the ring on the 64->64 layer
-    p.mcast = 1; p.TPS = 3; p.WST = 3 * p.nblk;
-  } else if (p.nsplit == 1 && 1024 + a_total + 2 * 3 * tap_bytes + 1024 <= half_sm) {
-    // multi-wave grids: 2-deep ring of 3-tap slabs (~105 KB) so TWO CTAs share an SM (256x256: 14.7 us vs 24.0 us)
-    p.TPS = 3; p.WST = 2;
-  } else if (p.nsplit == 1 && a_total + 2 * 3 * tap_bytes <= budget) {
-    p.TPS = 3; p.WST = (int)((budget - a_total) / (3 * tap_bytes));
-    if (p.WST > 3 * p.nblk) p.WST = 3 * p.nblk;
-    if (p.WST > MAX_WST) p.WST = MAX_WST;
-  } else {
-    p.TPS = 1;
-    int wst = (int)((budget - a_total) / tap_bytes);
-    if (wst > 9 * p.nblk) wst = 9 * p.nblk;
-    if (wst > MAX_WST) wst = MAX_WST;
-    TECO_CHECK_ARG(wst >= 2, "teco_conv3x3_tc(one-tile): shared memory budget too small (Cin=%d Cout=%d)", d->Cin, d->Cout);
-    p.WST = wst;
-  }
-  p.w_slab_bytes = (uint32_t)(p.TPS * tap_bytes);
-  p.KS = (p.TPS == 3 && d->mode == 0 && J * 3 * p.Ncta <= 512) ? 3 : 1;
-  p.CS = (p.mcast && p.num_tiles >= 8) ? 4 : 1;
-  uint32_t cols = (uint32_t)(J * nacc * p.KS * p.Ncta), tc = 32;
-  while (tc < cols) tc <<= 1;
-  p.tmem_cols = tc;
-  constexpr int env_tma = 1;   // staged (TMA-store) epilogue wherever the layer qualifies
-  p.tma_out = (env_tma && y && !out_f32 && p.Ncta == 64 &&
-               (d->mode == 0 || (!res && p.nsplit == 1 && d->H % TILE_ROWS == 0))) ? 1 : 0;   // tconv: rows of (n, y) are one map dimension
-  p.tma_res = (p.tma_out && res) ? 1 : 0;
-  p.stage2_bytes = p.tma_res ? (uint32_t)(J * 16384) : ((p.tma_out && d->mode == 1) ? 16384u : 0u);
-  TECO_CHECK_ARG(!p.tma_out || (size_t)J * 16384 <= a_total, "teco_conv3x3_tc(one-tile): output staging does not fit the halo stages");
-  const size_t smem_bytes = a_total + (size_t)p.WST * p.w_slab_bytes + p.stage2_bytes +
-                            (4 + 2 * MAX_WST + 2) * 8 + 256 * sizeof(float) + 16;
-  static const int env_late = [] { const char* e = getenv("TECO_TC_LATE_TRIGGER"); return e ? atoi(e) : 1; }();
-  p.late_trigger = (env_late && 2 * (smem_bytes + 1024) <= 228 * 1024) ? 1 : 0;   // only useful when two CTAs fit an SM
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) {
-    teco_set_error("teco_conv3x3_tc(one-tile): cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
-    return TECO_E_CUDA;
-  }
-  CUtensorMap tmap;
-  const cuuint64_t gdim[4] = {(cuuint64_t)d->Cin, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-  const cuuint64_t gstr[3] = {(cuuint64_t)d->Cin * 2, (cuuint64_t)d->W * d->Cin * 2, (cuuint64_t)d->H * d->W * d->Cin * 2};
-  const cuuint32_t box[4] = {(cuuint32_t)CB, (cuuint32_t)(H1 ? 8 * J + 2 : 8 * J), (cuuint32_t)HALO_ROWS, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), gdim, gstr, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) {
-    teco_set_error("teco_conv3x3_tc(one-tile): cuTensorMapEncodeTiled failed with CUresult %d (N=%d H=%d W=%d Cin=%d)", (int)cr, d->N,
-                   d->H, d->W, d->Cin);
-    return TECO_E_CUDA;
-  }
-  CUtensorMap tmap_y = tmap, tmap_r = tmap;   // placeholders when the staged epilogue is off
-  if (p.tma_out && d->mode == 1) {
-    // output [N, 2H, 2W, C] as {C, px, x, py, n*H + y}: one box = the 16x8 pixels of one sub-pixel phase
-    const cuuint64_t odim[5] = {(cuuint64_t)d->Cout, 2, (cuuint64_t)d->W, 2, (cuuint64_t)d->N * d->H};
-    const cuuint64_t ostr[4] = {(cuuint64_t)d->Cout * 2, (cuuint64_t)d->Cout * 4, (cuuint64_t)d->W * d->Cout * 4,
-                                (cuuint64_t)d->W * d->Cout * 8};
-    const cuuint32_t obox[5] = {64, 1, 8, 1, (cuuint32_t)TILE_ROWS};
-    const cuuint32_t estr5[5] = {1, 1, 1, 1, 1};
-    cr = enc(&tmap_y, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, y, odim, ostr, obox, estr5, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) {
-      teco_set_error("teco_conv3x3_tc(one-tile): cuTensorMapEncodeTiled (transposed-conv output) failed with CUresult %d", (int)cr);
-      return TECO_E_CUDA;
-    }
-  } else if (p.tma_out) {
-    const cuuint64_t odim[4] = {(cuuint64_t)d->Cout, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-    const cuuint64_t ostr[3] = {(cuuint64_t)d->Cout * 2, (cuuint64_t)d->W * d->Cout * 2, (cuuint64_t)d->H * d->W * d->Cout * 2};
-    const cuuint32_t obox[4] = {64, 8, (cuuint32_t)TILE_ROWS, 1};
-    cr = enc(&tmap_y, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, odim, ostr, obox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr == CUDA_SUCCESS && p.tma_res)
-      cr = enc(&tmap_r, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(res), odim, ostr, obox, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) {
-      teco_set_error("teco_conv3x3_tc(one-tile): cuTensorMapEncodeTiled (output tile) failed with CUresult %d", (int)cr);
-      return TECO_E_CUDA;
-    }
-  }
-  using KernelT = void (*)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const TcParams);
-  KernelT kern = nullptr;
-#define TECO_PICK(M, T, JJ, K)                                              \
-  if (d->mode == M && p.TPS == T && J == JJ && p.KS == K)                   \
-    kern = conv3x3_tc_kernel<M, T, JJ, K, 1>;
-  TECO_PICK(0, 3, 1, 3) TECO_PICK(0, 3, 2, 3) TECO_PICK(0, 3, 1, 1) TECO_PICK(0, 3, 2, 1) TECO_PICK(0, 1, 1, 1) TECO_PICK(0, 1, 2, 1)
-  TECO_PICK(1, 3, 1, 1) TECO_PICK(1, 3, 2, 1) TECO_PICK(1, 1, 1, 1) TECO_PICK(1, 1, 2, 1)
+  CUtensorMap maps[3];
+  if (int e = tc_encode_maps(pl, d, x, y, res, maps)) return e;
+  void (*kern)(CUtensorMap, CUtensorMap, CUtensorMap, TcParams) = nullptr;
+#define TECO_PICK(M, T, JJ, K) \
+  if (pl.kmode == M && pl.TPS == T && pl.J == JJ && pl.KS == K) kern = conv3x3_tc_onetile_kernel<M, T, JJ, K>;
+  // J = 2 needs >= 2 waves of 16-pixel-wide tiles: a conv that large is multi-wave and runs persistent, and a transposed
+  // conv that large always fits 3-tap slabs
+  TECO_PICK(0, 3, 1, 3) TECO_PICK(0, 3, 1, 1) TECO_PICK(0, 1, 1, 1)
+  TECO_PICK(1, 3, 1, 1) TECO_PICK(1, 3, 2, 1) TECO_PICK(1, 1, 1, 1)
 #undef TECO_PICK
   if (!kern) {
-    teco_set_error("teco_conv3x3_tc(one-tile): no kernel instantiation for mode=%d TPS=%d J=%d KS=%d", d->mode, p.TPS, J, p.KS);
+    teco_set_error("teco_conv3x3_tc(one-tile): no kernel instantiation for mode=%d TPS=%d J=%d KS=%d", pl.kmode, pl.TPS, pl.J, pl.KS);
     return TECO_E_UNSUPPORTED;
   }
-  TECO_CUDA_CALL(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(224 * 1024)));
-  p.tiles_pad = (p.num_tiles + p.CS - 1) / p.CS * p.CS;
-  const unsigned ctas = (unsigned)(p.tiles_pad * p.nsplit);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(ctas);
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = smem_bytes;
-  cfg.stream = (cudaStream_t)stream;
-  cudaLaunchAttribute attrs[2];
-  int na = 0;
-  attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // PDL: prologue overlaps the previous kernel's tail
-  attrs[na].val.programmaticStreamSerializationAllowed = 1;
-  ++na;
-  if (p.CS > 1) {
-    attrs[na].id = cudaLaunchAttributeClusterDimension;
-    attrs[na].val.clusterDim.x = (unsigned)p.CS;
-    attrs[na].val.clusterDim.y = 1;
-    attrs[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = attrs;
-  cfg.numAttrs = na;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, kern, tmap, tmap_y, tmap_r, p);
-  if (le != cudaSuccess) {
-    teco_set_error("teco_conv3x3_tc(one-tile): launch failed: %s (grid %u, cluster %d, smem %zu)", cudaGetErrorString(le), ctas, p.CS, smem_bytes);
-    return TECO_E_CUDA;
-  }
-  return TECO_OK;
+  return tc_launch(kern, 224 * 1024, NUM_THREADS, pl, maps, p, stream);
 }

@@ -134,20 +134,6 @@ conv3x3_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-PFN_encodeTiled wg_get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
-  return fn;
-}
-
 }  // namespace
 
 extern "C" int teco_conv3x3_wgrad_tc(int32_t N, int32_t H, int32_t W, int32_t cin_pad, int32_t cout_pad, int32_t cin, int32_t cout,
@@ -161,29 +147,9 @@ extern "C" int teco_conv3x3_wgrad_tc(int32_t N, int32_t H, int32_t W, int32_t ci
                  "teco_conv3x3_wgrad_tc: tensors must be 16-byte aligned");
   cudaStream_t s = (cudaStream_t)stream;
   if (!accumulate) TECO_CUDA_CALL(cudaMemsetAsync(dw, 0, sizeof(float) * (size_t)9 * cin * cout, s));
-  PFN_encodeTiled enc = wg_get_encode();
-  if (!enc) {
-    teco_set_error("teco_conv3x3_wgrad_tc: cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
-    return TECO_E_CUDA;
-  }
   CUtensorMap tx, tz;
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  {
-    const cuuint64_t gdim[4] = {(cuuint64_t)cin_pad, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-    const cuuint64_t gstr[3] = {(cuuint64_t)cin_pad * 2, (cuuint64_t)W * cin_pad * 2, (cuuint64_t)H * W * cin_pad * 2};
-    const cuuint32_t box[4] = {64, WG_COLS + 2, WG_ROWS + 2, 1};
-    CUresult cr = enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) { teco_set_error("teco_conv3x3_wgrad_tc: cuTensorMapEncodeTiled(x) failed with CUresult %d", (int)cr); return TECO_E_CUDA; }
-  }
-  {
-    const cuuint64_t gdim[4] = {(cuuint64_t)cout_pad, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-    const cuuint64_t gstr[3] = {(cuuint64_t)cout_pad * 2, (cuuint64_t)W * cout_pad * 2, (cuuint64_t)H * W * cout_pad * 2};
-    const cuuint32_t box[4] = {64, WG_COLS, WG_ROWS, 1};
-    CUresult cr = enc(&tz, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(dz), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) { teco_set_error("teco_conv3x3_wgrad_tc: cuTensorMapEncodeTiled(dz) failed with CUresult %d", (int)cr); return TECO_E_CUDA; }
-  }
+  if (int e = teco_tmap_nhwc(&tx, "teco_conv3x3_wgrad_tc (x)", x, N, H, W, cin_pad, 64, WG_COLS + 2, WG_ROWS + 2)) return e;
+  if (int e = teco_tmap_nhwc(&tz, "teco_conv3x3_wgrad_tc (dz)", dz, N, H, W, cout_pad, 64, WG_COLS, WG_ROWS)) return e;
   WgParams p;
   p.N = N; p.H = H; p.W = W; p.Cin = cin; p.Cout = cout;
   p.cob = teco_ceil_div(cout, 64);
@@ -194,11 +160,7 @@ extern "C" int teco_conv3x3_wgrad_tc(int32_t N, int32_t H, int32_t W, int32_t ci
   TECO_CHECK_ARG(tiles < (1LL << 31), "teco_conv3x3_wgrad_tc: too many tiles");
   const int cib = teco_ceil_div(cin, 64);
   const size_t smem = 1024 + ((WG_HALO_BYTES + 1023) & ~1023) + WG_DZ_BYTES + 64;
-  static bool attr = false;
-  if (!attr) {
-    TECO_CUDA_CALL(cudaFuncSetAttribute(conv3x3_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr = true;
-  }
+  TECO_CUDA_CALL(cudaFuncSetAttribute(conv3x3_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   conv3x3_wgrad_tc_kernel<<<dim3((unsigned)tiles, (unsigned)(cib * p.cob)), 128, smem, s>>>(tx, tz, p);
   TECO_CUDA_LAUNCH_CHECK("teco_conv3x3_wgrad_tc");
   return TECO_OK;

@@ -678,12 +678,8 @@ int teco_warp_s2d_fused(const float* pre_gen, const float* flow_lr, void* dst, f
   const int tiles_x = teco_ceil_div(w, WS_TLW), tiles_y = teco_ceil_div(h, WS_TLH);
   TECO_CHECK_ARG(tiles_y <= 65535 && N <= 65535, "teco_warp_s2d_fused: more than 65535 row bands or images");
   const size_t smem = WS_SMEM_FLOATS * sizeof(float);
-  static bool attr = false;
-  if (!attr) {
-    TECO_CUDA_CALL(cudaFuncSetAttribute(warp_s2d_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    TECO_CUDA_CALL(cudaFuncSetAttribute(warp_s2d_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr = true;
-  }
+  if (dst_bf16) TECO_CUDA_CALL(cudaFuncSetAttribute(warp_s2d_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  else TECO_CUDA_CALL(cudaFuncSetAttribute(warp_s2d_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // the 4-float stores of warped_out need 16-byte alignment of every (row, 4*lx) start: W*3 floats per row, 4*lx*3 = 12 lx
   TECO_CHECK_ARG(!warped_out || ((((uintptr_t)warped_out) & 15) == 0), "teco_warp_s2d_fused: warped_out must be 16-byte aligned");
   TECO_CHECK_ARG((((uintptr_t)pre_gen) & 15) == 0, "teco_warp_s2d_fused: pre_gen must be 16-byte aligned");

@@ -1,5 +1,6 @@
 // Shared helpers for libteco.so (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
@@ -35,6 +36,14 @@ void teco_set_error(const char* fmt, ...);
   } while (0)
 
 static inline int teco_ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
+
+// TMA tensor map over bf16 data with SWIZZLE_128B, 128-byte L2 promotion and zero fill out of bounds (TF 'SAME' padding
+// of the convolutions).  dims[0] is the contiguous dimension; strides[i] is the byte stride of dims[i + 1].  On failure
+// sets the error message, prefixed with `who`, and returns TECO_E_CUDA.
+int teco_tmap_bf16(CUtensorMap* map, const char* who, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                   const cuuint32_t* box);
+// The common case: NHWC [N][H][W][C] bf16, box = box_c channels x box_w pixels x box_h rows of one image.
+int teco_tmap_nhwc(CUtensorMap* map, const char* who, const void* base, int N, int H, int W, int C, int box_c, int box_w, int box_h);
 
 __device__ __forceinline__ float teco_act(float v, int act) {
   switch (act) {

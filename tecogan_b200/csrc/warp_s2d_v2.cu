@@ -292,11 +292,7 @@ bool teco_warp_s2d_v2_applicable(const void* dst, int dst_cpitch, int ch_off, in
 int teco_warp_s2d_v2_launch(const float* pre_gen, const float* flow_lr, void* dst, int N, int h, int w, int fh, int fw,
                             int dst_cpitch, int ch_off, float in_scale, float in_shift, cudaStream_t stream) {
   const size_t smem = V2_WIN_FLOATS * sizeof(float) + V2_STAGE_BYTES + sizeof(V2Smem);
-  static bool attr = false;
-  if (!attr) {
-    TECO_CUDA_CALL(cudaFuncSetAttribute(warp_s2d_v2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr = true;
-  }
+  TECO_CUDA_CALL(cudaFuncSetAttribute(warp_s2d_v2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int tiles_x = teco_ceil_div(w, V2_TLW), tiles_y = teco_ceil_div(h, V2_TLH);
   TECO_CHECK_ARG(tiles_y <= 65535 && N <= 65535, "teco_warp_s2d_fused: more than 65535 row bands or images");
   warp_s2d_v2_kernel<<<dim3((unsigned)tiles_x, (unsigned)tiles_y, (unsigned)N), V2_TPB, smem, stream>>>(

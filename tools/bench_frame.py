@@ -1,5 +1,5 @@
 """Frame rate of the streaming recurrence at LR 128x128 (configs[1]) with and without the fnet look-ahead.
-Usage: python tools/bench_frame.py [h w frames]   (env TECO_TC_H1 / TECO_TC_1CTA select conv kernel variants)"""
+Usage: python tools/bench_frame.py [h w frames]"""
 import os
 import sys
 
