@@ -246,6 +246,29 @@ int teco_metrics_psnr_y_u8(const uint8_t* tgt, int32_t tH, int32_t tW, const uin
 int teco_metrics_ssim_y_u8(const uint8_t* tgt, int32_t tH, int32_t tW, const uint8_t* out, int32_t oH, int32_t oW,
                            int32_t N, int32_t y0, int32_t x0, int32_t h, int32_t w, double* acc, void* stream);
 
+/* ---------------------------------------------------------------------------------------
+ * tOF (metrics.py:135-169): cv2.cvtColor(RGB2GRAY) and cv2.calcOpticalFlowFarneback with flags = 0 on the device,
+ * batched over all frame pairs of a scene.  The stages are pinned against cv2 in tests/golden/tof_ref.py.
+ * ------------------------------------------------------------------------------------- */
+/* grey[n][y][x] = (9798 R + 19235 G + 3735 B + 2^14) >> 15 (cv2's COLOR_RGB2GRAY on uint8, bit for bit) of the
+ * top-left h x w of frame n of rgb [N,H,W,3]: the reference's cut of the result to the target size, metrics.py:139-140. */
+int teco_grey_u8(const uint8_t* rgb, int32_t N, int32_t H, int32_t W, int32_t h, int32_t w, uint8_t* grey, void* stream);
+/* Host only: workspace bytes teco_farneback_flow needs for F frames and P pairs of H x W, or TECO_E_INVALID for bad sizes
+ * (F, P in 1..65535, H in 2..65535, W >= 2, H*W < 2^31, 0 < pyr_scale < 1, levels >= 0). */
+int64_t teco_farneback_workspace_bytes(int32_t F, int32_t P, int32_t H, int32_t W, double pyr_scale, int32_t levels);
+/* flow[p] = calcOpticalFlowFarneback(grey[pairs_host[2p]], grey[pairs_host[2p+1]], None, pyr_scale, levels, winsize,
+ * iterations, poly_n, poly_sigma, flags) for grey [F,H,W] uint8 and flow [P,H,W,2] float32 (dx, dy).  Each frame's
+ * polynomial expansion is computed once per level, however many pairs use it.  Supported: flags = 0, odd winsize up to 15,
+ * poly_n 1..7; anything else is TECO_E_INVALID.  pairs_host is read before the call returns.  A pair's flow is the same
+ * bits whatever else is in the batch. */
+int teco_farneback_flow(const uint8_t* grey, int32_t F, int32_t H, int32_t W, const int32_t* pairs_host, int32_t P,
+                        double pyr_scale, int32_t levels, int32_t winsize, int32_t iterations, int32_t poly_n,
+                        double poly_sigma, int32_t flags, void* workspace, int64_t workspace_bytes, float* flow, void* stream);
+/* sums[p] = sum over the window (y0,x0,h,w) of |flow_t[p] - flow_o[p]|_2 in float64, both [P,H,W,2]; tOF_p = sums[p] / (h*w).
+ * Overwrites sums; no atomics, so the result does not depend on scheduling. */
+int teco_tof_sums(const float* flow_t, const float* flow_o, int32_t P, int32_t H, int32_t W, int32_t y0, int32_t x0,
+                  int32_t h, int32_t w, double* sums, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -3,10 +3,11 @@
 metrics that are image arithmetic: PSNR and SSIM on the Y channel, computed on the GPU by tecogan_b200/metrics.py
 (teco_metrics_psnr_y_u8 / teco_metrics_ssim_y_u8).  Same frame selection (cutfr = 2, metrics.py:117,131), same cut of the
 result to the target size (:134-135), same crop_8x8 (:171-172), same per-frame / per-folder / total printout and
-metrics.csv layout (:205-242) restricted to keys = ["PSNR", "SSIM"].
-LPIPS / tLP (AlexNet weights) and tOF (cv2 Farneback on the CPU) are not part of this path: DESIGN.md section 6.
+metrics.csv layout (:205-242) for the keys named by --keys (the reference's `keys` list, :120): PSNR and SSIM by default,
+tOF on request (cv2's Farneback flow, metrics.py:135-169, as the CUDA kernels of tecogan_b200/csrc/optflow.cu).
+LPIPS / tLP (AlexNet weights not available) are not part of this path: DESIGN.md section 6.
 
-  python metrics.py --output results/metric_log/ --results results/calendar --targets HR/calendar
+  python metrics.py --output results/metric_log/ --results results/calendar --targets HR/calendar [--keys PSNR,SSIM,tOF]
 """
 import argparse
 import os
@@ -18,7 +19,17 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 
 KEYS = ["PSNR", "SSIM"]
+KNOWN_KEYS = ("PSNR", "SSIM", "tOF")
 CUTFR = 2
+
+
+def parse_keys(text):
+    """--keys: comma-separated subset of PSNR, SSIM, tOF; kept in the reference's order (metrics.py:120)."""
+    keys = [k.strip() for k in text.split(",") if k.strip()]
+    bad = [k for k in keys if k not in KNOWN_KEYS]
+    if bad or not keys:
+        raise ValueError("--keys: unknown or empty %s (known: %s)" % (bad or text, ",".join(KNOWN_KEYS)))
+    return [k for k in KNOWN_KEYS if k in keys]
 
 
 def listPNGinDir(dirpath):
@@ -37,8 +48,10 @@ def read_rgb(path):
         return np.ascontiguousarray(np.asarray(Image.open(path).convert("RGB")))
 
 
-def evaluate_folder(result_dir, target_dir, log=print):
-    """Per-frame PSNR / SSIM lists of one scene (frames cutfr .. n-cutfr-1), frames grouped by size into batched launches."""
+def evaluate_folder(result_dir, target_dir, log=print, keys=KEYS):
+    """Per-frame lists of one scene (frames cutfr .. n-cutfr-1) for `keys`."""
+    if "tOF" in keys:
+        return _evaluate_folder_batched(result_dir, target_dir, log, keys)
     import torch
     from tecogan_b200 import metrics as M
     result, target = listPNGinDir(result_dir), listPNGinDir(target_dir)
@@ -56,12 +69,49 @@ def evaluate_folder(result_dir, target_dir, log=print):
     return lists
 
 
+def _evaluate_folder_batched(result_dir, target_dir, log, keys):
+    """The folder loaded once, tOF of all frame pairs in one batched call, PSNR / SSIM of all frames in one batch; the
+    per-frame lines follow metrics.py:169-185 (tOF before psnr, none on the first frame)."""
+    import torch
+    from tecogan_b200 import metrics as M
+    result, target = listPNGinDir(result_dir), listPNGinDir(target_dir)
+    idx = list(range(CUTFR, len(target) - CUTFR))
+    tars = [read_rgb(target[i]) for i in idx]
+    outs = [read_rgb(result[i]) for i in idx]
+    th, tw = tars[0].shape[:2]
+    if any(t.shape != tars[0].shape for t in tars) or any(o.shape[0] < th or o.shape[1] < tw for o in outs):
+        raise ValueError("%s: tOF needs target frames of one size and result frames at least that large" % target_dir)
+    t = torch.from_numpy(np.stack(tars)).cuda()
+    o = torch.from_numpy(np.stack([x[:th, :tw] for x in outs])).cuda()      # metrics.py:139-140
+    tof = M.tof(t, o, cutfr=0)
+    ps, ss = M.frame_metrics(t, o) if ("PSNR" in keys or "SSIM" in keys) else ([], [])
+    y, x, _, _ = M.crop_window(th, tw)
+    lists = {"PSNR": ps, "SSIM": ss, "tOF": tof}
+    for j, i in enumerate(idx):
+        msg = "frame %d, tar %s, out %s, " % (i, str(tars[j].shape), str(outs[j].shape))
+        if j > 0:
+            msg += "tOF %02.2f, " % tof[j - 1]
+        parts = []
+        if "PSNR" in keys:
+            parts.append("psnr %02.2f" % ps[j])
+        if "SSIM" in keys:
+            parts.append("ssim %02.2f" % ss[j])
+        log(result[i])
+        log(msg + ", ".join(parts + ["crop (%d, %d)" % (y, x)]))
+    return {k: lists[k] for k in keys}
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--output", required=True, help="the path of output directory")
     ap.add_argument("--results", required=True, help="the list of paths of result directory")
     ap.add_argument("--targets", required=True, help="the list of paths of target directory")
+    ap.add_argument("--keys", default="PSNR,SSIM", help="comma-separated metrics out of PSNR, SSIM, tOF")
     F = ap.parse_args(argv)
+    try:
+        keys = parse_keys(F.keys)
+    except ValueError as e:
+        ap.error(str(e))
     import pandas as pd
     os.makedirs(F.output, exist_ok=True)
     logf = open(os.path.join(F.output, "metricsfile.txt"), "a")
@@ -71,15 +121,15 @@ def main(argv=None):
         logf.write(m + "\n")
     result_list, target_list = F.results.split(','), F.targets.split(',')
     folder_n = len(result_list)
-    sum_d = {"FrameAvg_" + k: 0.0 for k in KEYS}
-    len_d = {k: 0 for k in KEYS}
-    avg_d = {"Avg_" + k: [] for k in KEYS}
-    folder_d = {"FolderAvg_" + k: 0.0 for k in KEYS}
+    sum_d = {"FrameAvg_" + k: 0.0 for k in keys}
+    len_d = {k: 0 for k in keys}
+    avg_d = {"Avg_" + k: [] for k in keys}
+    folder_d = {"FolderAvg_" + k: 0.0 for k in keys}
     csv = os.path.join(F.output, "metrics.csv")
     for fi in range(folder_n):
-        lists = evaluate_folder(result_list[fi], target_list[fi], log)
+        lists = evaluate_folder(result_list[fi], target_list[fi], log, keys)
         pd_dict = {}
-        for k in KEYS:
+        for k in keys:
             cur = np.float32(lists[k])
             pd_dict["%s_%02d" % (k, fi)] = pd.Series(cur)
             mean = cur.sum() / cur.shape[0]
@@ -89,7 +139,7 @@ def main(argv=None):
             len_d[k] += cur.shape[0]
             folder_d["FolderAvg_" + k] += mean
         pd.DataFrame(pd_dict).to_csv(csv, mode='w' if fi == 0 else 'a')
-    for k in KEYS:
+    for k in keys:
         sum_d["FrameAvg_" + k] = pd.Series([sum_d["FrameAvg_" + k] / len_d[k]])
         folder_d["FolderAvg_" + k] = pd.Series([folder_d["FolderAvg_" + k] / folder_n])
         avg_d["Avg_" + k] = pd.Series(np.float32(avg_d["Avg_" + k]))
@@ -98,7 +148,7 @@ def main(argv=None):
         pd.DataFrame(d).to_csv(csv, mode='a')
     log("Finished.")
     logf.close()
-    return {k: float(sum_d["FrameAvg_" + k][0]) for k in KEYS}
+    return {k: float(sum_d["FrameAvg_" + k][0]) for k in keys}
 
 
 if __name__ == "__main__":

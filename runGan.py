@@ -4,8 +4,8 @@ Mirror of the reference's runGan.py launcher (run cases, reference runGan.py:1-1
 python3 runGan.py 1   # inference on LR/calendar with the flags of record (reference runGan.py:67-90)
 python3 runGan.py 3   # train TecoGAN  (reference runGan.py:107-244)
 python3 runGan.py 4   # train FRVSR    (reference runGan.py:247-296)
-python3 runGan.py 2   # PSNR / SSIM of ./results/<scene> against ./HR/<scene> on the GPU (reference runGan.py:92-105; the
-                      # LPIPS / tLP / tOF columns of the reference's metrics.py are outside the hot path, DESIGN.md section 6)
+python3 runGan.py 2   # PSNR / SSIM of ./results/<scene> against ./HR/<scene> on the GPU (reference runGan.py:92-105; tOF
+                      # is available through `metrics.py --keys PSNR,SSIM,tOF`; LPIPS / tLP are not, DESIGN.md section 6)
 Case 0 (download, needs network) is outside the hot path and prints why it is not run.
 Extra arguments after the case number are appended to the main.py command line (e.g. --max_iter 100).
 '''

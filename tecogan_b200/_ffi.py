@@ -29,7 +29,7 @@ class TcDesc(C.Structure):
         ("post_scale", C.c_float), ("post_shift", C.c_float)]
 
 
-_P, _I32, _I64, _F = C.c_void_p, C.c_int32, C.c_int64, C.c_float
+_P, _I32, _I64, _F, _D = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 
 # symbol -> argtypes (restype is int unless listed in _RESTYPES).  Mirrors include/teco.h one to one;
 # tests/test_abi.py checks this table against the header and against the built library.
@@ -79,8 +79,12 @@ SIGNATURES = {
     "teco_adam_f32": [_P, _P, _P, _P, _I64, _F, _F, _F, _F, _F, _P],
     "teco_metrics_psnr_y_u8": [_P, _I32, _I32, _P, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P],
     "teco_metrics_ssim_y_u8": [_P, _I32, _I32, _P, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P],
+    "teco_grey_u8": [_P, _I32, _I32, _I32, _I32, _I32, _P, _P],
+    "teco_farneback_workspace_bytes": [_I32, _I32, _I32, _I32, _D, _I32],
+    "teco_farneback_flow": [_P, _I32, _I32, _I32, _P, _I32, _D, _I32, _I32, _I32, _I32, _D, _I32, _P, _I64, _P, _P],
+    "teco_tof_sums": [_P, _P, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P],
 }
-_RESTYPES = {"teco_packed_weight_bytes": C.c_int64, "teco_crc32c": C.c_int64}
+_RESTYPES = {"teco_packed_weight_bytes": C.c_int64, "teco_crc32c": C.c_int64, "teco_farneback_workspace_bytes": C.c_int64}
 
 _lib = None
 
